@@ -29,6 +29,7 @@ sys.path.insert(0, ROOT)
 
 A_GET = 16 + (16 + 64 + 8) + 64          # algorithmic bytes per MultiGet hit (SURVEY §8d)
 A_PUT = 83 + 22 + 88                     # per single-Put apply
+DUMP_LOOKUPS = 65536                     # MultiGet results kept by --dump-outputs: 65536 x 64 values = 16 MB as float32
 
 
 def peaks():
@@ -102,9 +103,9 @@ class ClockSampler:
 
 
 def run_cpu(lib_kind, threads, shards, kv, apply_cap, get_secs, batch=4096, wal=1):
-    """times oracle/okv_cpu_bench (the reference's RocksDB binary when oracle/_ref is present, else the port)"""
+    """times oracle/okv_cpu_bench (the reference's RocksDB binary when build() left it in oracle/_ref, else the port)"""
     from oracle import okv
-    okv.build(ref=os.path.isdir("/root/reference"))
+    okv.build(ref=False)
     lib = okv.REF_SO if (lib_kind == "reference" and okv.ref_available()) else okv.PORT_SO
     base = "/dev/shm" if os.path.isdir("/dev/shm") else "/tmp"
     d = os.path.join(base, "okv_bench_%d" % os.getpid())
@@ -183,7 +184,13 @@ def main():
     ap.add_argument("--cpu-get-secs", type=float, default=6.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-seams", action="store_true", help="skip the through-the-seams phase (librsp_host.so)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed step returned the last time as DIR/<name>.npy (float32 / float64, rank 0): "
+                         "MultiGet values, lengths and statuses of a fixed sample of %d lookups, and the apply tick's "
+                         "per-batch statuses; the same arguments give the same inputs" % DUMP_LOOKUPS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm returns no arrays")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -313,6 +320,13 @@ def main():
     want = synth.values(seed, (last % np.uint64(S)).astype(np.int64), last, 0)
     got = d_vals.cpu().numpy().reshape(Q, 64)
     assert np.array_equal(got, want), "MultiGet parity failed at full size"
+    dump = {}
+    if args.dump_outputs:  # the later phases reuse these buffers: sample them now
+        rows = np.sort(np.random.default_rng(0).choice(Q, size=min(Q, DUMP_LOOKUPS), replace=False))
+        dump["multiget_lookup_index"] = rows.astype(np.float64)
+        dump["multiget_values"] = got[rows].astype(np.float32)
+        dump["multiget_value_len"] = d_vlen.cpu().numpy()[rows].astype(np.float32)
+        dump["multiget_status"] = d_st.cpu().numpy()[rows].astype(np.float32)
 
     # ---- config-2 variant: 10 % of the lookups ask for keys that were never written (NotFound) ------------
     with torch.cuda.stream(stream):
@@ -504,6 +518,8 @@ def main():
     ap_kernel_ms = eng.last_kernel_ms("apply")
     ap_launches = eng.kernel_launches() - launches1
     assert not st_out.any()
+    if args.dump_outputs:  # fold() read the last tick's statuses last
+        dump["apply_status"] = st_out.astype(np.float32)
 
     for stp in range(n_sets):
         ver_of[upd_idx[stp].astype(np.int64)] = stp + 1
@@ -898,6 +914,10 @@ def main():
             "clocks": clk,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     for h in staged:
         lib.rsp_stage_free(h)
     eng.close()

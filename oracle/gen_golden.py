@@ -1,15 +1,19 @@
-"""Generate tests/golden/*.json from the reference's OWN RocksDB binary (oracle/_ref).
+"""Generate tests/golden/*.json and tests/golden/ref_written_*.sst from the reference's OWN RocksDB binary (oracle/_ref).
 
-Run in the build container (needs oracle/_ref, i.e. /root/reference at build time):
+Needs oracle/_ref, which `make -C oracle ref` builds from the reference's sources:
     python -m oracle.gen_golden
-The fixtures pin the oracle port (tests/test_oracle_golden.py) and the CUDA engine (tests/test_parity_gpu.py)
-to outputs of the reference itself; they travel to the GPU box, /root/reference does not.
+The fixtures pin the oracle port (tests/test_oracle_golden.py), the SST reader / writer (tests/test_sst_cpu.py) and the
+CUDA engine (tests/test_parity_gpu.py, tests/test_zz_ingest_gpu.py) to outputs of the reference itself, so the tests
+need neither the reference nor its binary.
 TEST INFRASTRUCTURE ONLY.
 """
+import ctypes as C
 import json
 import os
+import shutil
 import struct
 import sys
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -17,7 +21,9 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from oracle import okv  # noqa: E402
+from golden_util import digest, sha256  # noqa: E402
 from streams import corrupt_cases, random_stream  # noqa: E402
+from rocksplicator_b200 import sst  # noqa: E402
 from rocksplicator_b200.write_batch import WriteBatch  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -140,13 +146,125 @@ def gen_known_answers(ref):
     return rows
 
 
+def _sst_api(ref):
+    ref.okv_write_sst.restype = C.c_int
+    ref.okv_write_sst.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_void_p, C.c_char_p, C.c_void_p, C.c_char_p, C.c_size_t]
+    ref.okv_ingest_sst.restype = C.c_int
+    ref.okv_ingest_sst.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_char_p, C.c_size_t]
+
+
+def _ingest(ref, db, tmp, data, allow=True):
+    """-> (rc, error text, path of the ingested file)"""
+    path = os.path.join(tmp, "f%d.sst" % len(os.listdir(tmp)))
+    with open(path, "wb") as f:
+        f.write(data)
+    err = C.create_string_buffer(256)
+    rc = ref.okv_ingest_sst(db.h, path.encode(), 1 if allow else 0, err, 256)
+    return rc, err.value.decode(), path
+
+
+def gen_ref_written(ref):
+    """tests/golden/ref_written_<n>.sst: the reference's SstFileWriter on test_sst_cpu.REF_WRITTEN"""
+    import numpy as np
+    from test_sst_cpu import REF_WRITTEN, _kv
+    for n, seed, max_v in REF_WRITTEN:
+        kv = _kv(n, seed, max_v=max_v)
+        koff = np.zeros(len(kv) + 1, dtype=np.uint64)
+        voff = np.zeros(len(kv) + 1, dtype=np.uint64)
+        np.cumsum([len(k) for k, _ in kv], out=koff[1:])
+        np.cumsum([len(v) for _, v in kv], out=voff[1:])
+        path = os.path.join(OUT, "ref_written_%d.sst" % n)
+        err = C.create_string_buffer(256)
+        rc = ref.okv_write_sst(path.encode(), len(kv), b"".join(k for k, _ in kv) + b"\0", koff.ctypes.data,
+                               b"".join(v for _, v in kv) + b"\0", voff.ctypes.data, err, 256)
+        assert rc == 0, err.value
+        print(os.path.basename(path), os.path.getsize(path), "bytes")
+
+
+def gen_sst_ingest(ref, tmp):
+    """test_sst_cpu.test_reference_ingests_files_written_here: the reference ingesting the files our writer produces"""
+    from test_sst_cpu import INGESTED, ingest_inputs
+    out = {}
+    for n, seed in INGESTED:
+        kv, kv2 = ingest_inputs(n, seed)
+        f1, f2 = sst.write_sst(kv), sst.write_sst(kv2)
+        db = okv.Okv(ref)
+        rc, error, _ = _ingest(ref, db, tmp, f1)
+        r = {"file": sha256(f1), "rc": rc, "error": error, "seq": db.latest_seq(), "scan": digest(db.scan()),
+             "get": digest([db.get(k) for k, _ in kv[:: max(1, len(kv) // 50)]])}
+        rc, error, path2 = _ingest(ref, db, tmp, f2)
+        with open(path2, "rb") as f:
+            after = f.read()
+        r.update({"file2": sha256(f2), "rc2": rc, "error2": error, "seq2": db.latest_seq(), "scan2": digest(db.scan()),
+                  "file2_after": sha256(after)})
+        db.close()
+        out[str(n)] = r
+    return out
+
+
+def gen_ingest_gpu(ref, tmp):
+    """test_zz_ingest_gpu.test_ingest_sequence_rules_and_contents: the reference's answers, call by call (RecordedRef)"""
+    from test_zz_ingest_gpu import ingest_inputs
+    f1, wb1, f2, f3, f4, wb2 = ingest_inputs()
+    db = okv.Okv(ref)
+    out = []
+
+    def ingest(kv, allow=True):
+        data = sst.write_sst(kv)
+        out.append(["ingest", sha256(data), int(allow), _ingest(ref, db, tmp, data, allow)[0]])
+
+    def apply(batch):
+        out.append(["apply", sha256(batch), 1234, db.apply(batch, 1234)])
+
+    def check():
+        out.append(["check", db.latest_seq(), digest(db.scan())])
+
+    ingest(f1), check()
+    apply(wb1), check()
+    ingest(f2), check()
+    ingest(f3), check()
+    ingest(f4, allow=False), check()
+    apply(wb2), check()
+    check()  # after the shard's full compaction
+    check()  # after the two unsorted files it refuses
+    db.close()
+    return out
+
+
+def gen_differential(ref):
+    """The reference's side of the differential tests, as digests (golden_util.digest) of what it returned"""
+    from oracle import fuzz_corrupt_port_vs_ref as fzc
+    from oracle import fuzz_port_vs_ref as fz
+    from test_oracle_golden import live_observations
+    pre = WriteBatch().put(b"pre", b"x").data()
+    corrupt = {}
+    for seed in range(0, 25):
+        mop, cs = fzc.cases(seed)
+        corrupt[str(seed)] = []
+        for bt, ts in cs:
+            db = okv.Okv(ref, merge_op=mop)
+            corrupt[str(seed)].append(fzc.recorded_outcome(fzc.outcome(db, pre, bt, ts)))
+            db.close()
+    tmp = tempfile.mkdtemp()
+    try:
+        return {"live": [digest(o) for o in live_observations(ref, ref_side=True)],
+                "fuzz": {str(s): [digest(o) for o in fz.observe(s, ref)] for s in range(200, 212)},
+                "corrupt_fuzz": corrupt,
+                "sst_ingest": gen_sst_ingest(ref, tmp),
+                "ingest_gpu": gen_ingest_gpu(ref, tmp)}
+    finally:
+        shutil.rmtree(tmp)
+
+
 def main():
     if not okv.ref_available():
-        raise SystemExit("oracle/_ref not built: run `make -C oracle ref` where /root/reference exists")
+        raise SystemExit("oracle/_ref not built: run `make -C oracle ref` with the reference's sources at REF")
     ref = okv.load_ref()
+    _sst_api(ref)
     os.makedirs(OUT, exist_ok=True)
+    gen_ref_written(ref)
     for name, data in (("streams.json", gen_streams(ref)), ("corrupt.json", gen_corrupt(ref)),
-                       ("known_answers.json", gen_known_answers(ref))):
+                       ("known_answers.json", gen_known_answers(ref)), ("differential.json", gen_differential(ref))):
         with open(os.path.join(OUT, name), "w") as f:
             json.dump({"generator": "oracle/gen_golden.py", "source": "rocksdb_admin/tests/librocksdb.so.5.4",
                        "cases": data}, f, separators=(",", ":"))

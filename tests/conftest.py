@@ -16,16 +16,8 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def port_lib():
     from oracle import okv
-    okv.build(ref=os.path.isdir("/root/reference"))
+    okv.build(ref=False)
     return okv.load_port()
-
-
-@pytest.fixture(scope="session")
-def ref_lib(port_lib):
-    from oracle import okv
-    if not okv.ref_available():
-        pytest.skip("oracle/_ref (the reference's own RocksDB binary) not built here")
-    return okv.load_ref()
 
 
 @pytest.fixture(scope="session", autouse=True)

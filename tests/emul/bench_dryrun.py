@@ -3,7 +3,7 @@ device + e2e, the mixed phase, the full-size parity assertions, the JSON line) o
 an edit to bench.py or an API drift is caught without a GPU.  torch.cuda is replaced by no-op stand-ins (emulated
 "device" pointers are host pointers, so CPU tensors serve as device buffers); timings are meaningless and ignored.
 
-    python tests/emul/bench_dryrun.py            # prints the JSON line bench.py would print
+    python tests/emul/bench_dryrun.py [bench.py arguments]   # prints the JSON line bench.py would print
 """
 import contextlib
 import os
@@ -82,10 +82,11 @@ def main(argv=None):
     spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
-    sys.argv = ["bench.py"] + (argv or ["--shards", "8", "--kv", "6000", "--mg-batches", "1", "--tick", "5", "--steps", "2",
-                                        "--warmup", "1", "--no-cpu", "--big-tick", "40", "--c5-secs", "0.5"])
+    # arguments given here come after the toy-size defaults, so they add to them or override them
+    sys.argv = ["bench.py", "--shards", "8", "--kv", "6000", "--mg-batches", "1", "--tick", "5", "--steps", "2",
+                "--warmup", "1", "--no-cpu", "--big-tick", "40", "--c5-secs", "0.5"] + (argv or [])
     bench.main()
 
 
 if __name__ == "__main__":
-    main(sys.argv[1:] or None)
+    main(sys.argv[1:])

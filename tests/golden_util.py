@@ -4,6 +4,7 @@ A "db" is anything with the Okv method set: apply(batch, ts) -> rc, latest_seq()
 multi_get(keys) -> [(rc, v)], scan(start=None, limit=None), iterator() (seek/seek_to_last/next/prev/
 valid/key/value/status/close), flush(), compact(), last_error.
 """
+import hashlib
 import json
 import os
 
@@ -18,6 +19,16 @@ def load(name):
 
 def unhex(x):
     return None if x is None else bytes.fromhex(x)
+
+
+def digest(obj):
+    """Short stable fingerprint of an observation (nested tuples / lists of bytes, str, int, bool, None): lets the
+    golden files hold what the reference returned for large results without storing the results themselves."""
+    return hashlib.sha256(repr(obj).encode()).hexdigest()[:16]
+
+
+def sha256(data):
+    return hashlib.sha256(data).hexdigest()
 
 
 def check_snapshot(db, keys, snap, tag=""):

@@ -80,14 +80,15 @@ def test_engine_vs_oracle_corruption_fuzz_under_emulation(emul):
     assert p.returncode == 0 and "done bad= 0" in p.stdout
 
 
-def test_bench_control_flow_under_emulation(emul):
+def test_bench_control_flow_under_emulation(emul, tmp_path):
     """bench.py end to end at toy size (tests/emul/bench_dryrun.py): every phase, its own full-size parity assertions
     and the JSON contract keys — an edit to bench.py or an API drift shows up here, not on the GPU box"""
     import json
     env = dict(os.environ)
     env["RSP_TEST_EMUL_LIB"] = emul[0]
-    p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emul", "bench_dryrun.py")], cwd=ROOT, env=env,
-                       capture_output=True, text=True, timeout=900)
+    dump = tmp_path / "outputs"
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emul", "bench_dryrun.py"), "--dump-outputs", str(dump)],
+                       cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
     print(p.stdout[-1500:], p.stderr[-2500:])
     assert p.returncode == 0
     line = json.loads(p.stdout.strip().splitlines()[-1])
@@ -100,6 +101,20 @@ def test_bench_control_flow_under_emulation(emul):
     assert set(line["e2e"]) >= {"value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step"}
     assert "error" not in line["memtable"] and line["memtable"]["lookups_per_s"] > 0 and line["memtable"]["memtable_entries"] > 0
     assert "error" not in line["two_runs"] and line["two_runs"]["lookups_per_s"] > 0 and "2 sorted runs" in line["two_runs"]["what"]
+    # --dump-outputs: the last timed step's results (bench_dryrun's toy size: 8 shards, 6000 KV, one MultiGet(4096) and
+    # 8 x 5 batches per step, 1 warm-up + 2 timed steps), as float arrays
+    import numpy as np
+    from rocksplicator_b200 import synth
+    out = {f.stem: np.load(f) for f in dump.glob("*.npy")}
+    assert set(out) == {"multiget_lookup_index", "multiget_values", "multiget_value_len", "multiget_status", "apply_status"}
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(f.stat().st_size for f in dump.glob("*.npy")) <= 64 << 20
+    rng = np.random.default_rng(synth.SEED_QUERY)
+    last = [rng.integers(0, 6000, size=4096, dtype=np.uint64) for _ in range(3)][-1]
+    assert np.array_equal(out["multiget_lookup_index"], np.arange(4096))
+    assert np.array_equal(out["multiget_values"], synth.values(synth.SEED_DATA, (last % np.uint64(8)).astype(np.int64), last, 0))
+    assert (out["multiget_value_len"] == 64).all() and (out["multiget_status"] == 0).all()
+    assert out["apply_status"].shape == (8 * 5,) and (out["apply_status"] == 0).all()
 
 
 def test_host_mirror_over_emulated_engine(emul):

@@ -1,7 +1,8 @@
 """Pins the oracle port (oracle/kv_oracle.c) to the reference:
   1. known-answer table measured on the reference's shipped librocksdb.so.5.4 (SURVEY.md §9),
   2. tests/golden/*.json generated from that binary by oracle/gen_golden.py,
-  3. live differential runs against the binary when oracle/_ref is present (build container).
+  3. differential runs (random streams, fuzzers) against the binary's results for the same calls, recorded by
+     oracle/gen_golden.py in tests/golden/differential.json.
 CPU only.
 """
 import struct
@@ -111,52 +112,63 @@ def test_replicator_test_vectors(port_lib):
     db.close()
 
 
-def test_port_vs_reference_live(port_lib, ref_lib):
-    """Differential: fresh random streams (not in the fixtures) through both."""
+def live_observations(lib, ref_side):
+    """The calls of test_port_vs_reference_live and what `lib` returns for each.  On the reference's side the stream
+    is flushed after batch 40 and compacted at the end: the results must not depend on that."""
+    out = []
     for mop, mname in ((okv.MERGE_COUNTER, "counter"), (okv.MERGE_APPEND, "append")):
         for seed in (91, 92):
             keys, stream = random_stream(seed + mop, 80, merge=mname)
-            a = okv.Okv(port_lib, merge_op=mop)
-            b = okv.Okv(ref_lib, merge_op=mop)
+            db = okv.Okv(lib, merge_op=mop)
             for i, (bt, ts) in enumerate(stream):
-                assert a.apply(bt, ts) == b.apply(bt, ts)
-                if i == 40:
-                    b.flush()
-            b.compact()
-            assert a.latest_seq() == b.latest_seq()
-            for k in keys:
-                assert a.get(k) == b.get(k)
-            assert a.multi_get(keys) == b.multi_get(keys)
-            assert a.scan() == b.scan()
-            a.close()
-            b.close()
+                out.append(db.apply(bt, ts))
+                if ref_side and i == 40:
+                    db.flush()
+            if ref_side:
+                db.compact()
+            out.append((db.latest_seq(), [db.get(k) for k in keys], db.multi_get(keys), db.scan()))
+            db.close()
     for name, bt in corrupt_cases():
-        a = okv.Okv(port_lib, merge_op=okv.MERGE_UINT64ADD)
-        b = okv.Okv(ref_lib, merge_op=okv.MERGE_UINT64ADD)
-        assert a.apply(bt, 7) == b.apply(bt, 7), name
-        assert a.last_error == b.last_error, name
-        assert a.latest_seq() == b.latest_seq(), name
-        a.close()
-        b.close()
+        db = okv.Okv(lib, merge_op=okv.MERGE_UINT64ADD)
+        out.append((name, db.apply(bt, 7), db.last_error, db.latest_seq()))
+        db.close()
+    return out
 
 
-def test_port_vs_reference_fuzz(port_lib, ref_lib):
-    """oracle/fuzz_port_vs_ref.py on a few seeds: flush/compaction at random points, MultiGet, iterator walks."""
+def test_port_vs_reference_live(port_lib):
+    """Differential: random streams (not in the fixtures) through the port against the reference's results for the
+    same calls (tests/golden/differential.json, recorded by oracle/gen_golden.py)."""
+    want = G.load("differential.json")["live"]
+    got = [G.digest(o) for o in live_observations(port_lib, ref_side=False)]
+    assert len(got) == len(want)
+    assert [i for i, (g, w) in enumerate(zip(got, want)) if g != w] == []
+
+
+def _oracle_module(name):
     import importlib.util
     import os
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "fuzz_port_vs_ref.py")
-    spec = importlib.util.spec_from_file_location("fuzz_port_vs_ref", path)
+    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", name + ".py")
+    spec = importlib.util.spec_from_file_location(name, path)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
-    assert mod.run(200, 212, port_lib, ref_lib) == 0
+    return mod
 
 
-def test_port_vs_reference_corruption_fuzz(port_lib, ref_lib):
-    """oracle/fuzz_corrupt_port_vs_ref.py on a few seeds: mutated batches, error class + text + latch + contents"""
-    import importlib.util
-    import os
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "fuzz_corrupt_port_vs_ref.py")
-    spec = importlib.util.spec_from_file_location("fuzz_corrupt_port_vs_ref", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    assert mod.run(0, 25, port_lib, ref_lib) == 0
+def test_port_vs_reference_fuzz(port_lib):
+    """oracle/fuzz_port_vs_ref.py on a few seeds: flush/compaction at random points, MultiGet, iterator walks; every
+    observation against the reference's (tests/golden/differential.json)."""
+    mod = _oracle_module("fuzz_port_vs_ref")
+    want = G.load("differential.json")["fuzz"]
+    assert sorted(want, key=int) == [str(s) for s in range(200, 212)]
+    for seed in range(200, 212):
+        got = [G.digest(o) for o in mod.observe(seed, port_lib)]
+        assert got == want[str(seed)], seed
+
+
+def test_port_vs_reference_corruption_fuzz(port_lib):
+    """oracle/fuzz_corrupt_port_vs_ref.py on a few seeds: mutated batches, error class + text + latch + contents, against
+    the reference's outcomes (tests/golden/differential.json)"""
+    mod = _oracle_module("fuzz_corrupt_port_vs_ref")
+    recorded = G.load("differential.json")["corrupt_fuzz"]
+    assert sorted(recorded, key=int) == [str(s) for s in range(0, 25)]
+    assert mod.run(0, 25, port_lib, recorded=recorded) == 0

@@ -1,19 +1,25 @@
 """SST interchange on the host (SURVEY §8f rank 2), CPU only.
   * the reference's golden file rocksdb_admin/tests/old_sst_data.sst (copied byte-for-byte to tests/golden/: a 978-byte
     test fixture, Snappy-compressed block) must read as key0..key9 -> value0..value9 (sst_binary.cpp:43-58);
-  * files written by the reference's own SstFileWriter (librocksdb.so.5.4) must read back exactly;
+  * files written by the reference's own SstFileWriter (librocksdb.so.5.4, stored under tests/golden/) must read back
+    exactly;
   * files written by OUR writer must be accepted by the reference's DB::IngestExternalFile and scan back exactly,
-    with the sequence-number rule of rocksdb_assumption_test.cpp:248-262 (ingest into an empty DB: seq stays 0)."""
-import ctypes as C
+    with the sequence-number rule of rocksdb_assumption_test.cpp:248-262 (ingest into an empty DB: seq stays 0).
+The reference's side of both was recorded by oracle/gen_golden.py."""
 import os
 import random
 import tempfile
 
 import pytest
 
+import golden_util as G
 from rocksplicator_b200 import sst
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "old_sst_data.sst")
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLDEN = os.path.join(GOLDEN_DIR, "old_sst_data.sst")
+# (n, seed, max_v) of the files the reference wrote and tests/golden/ stores: the many-block file has short values to
+# stay under 100 KB
+REF_WRITTEN = ((1, 11, 2000), (50, 12, 2000), (2000, 13, 8))
 
 
 def test_golden_old_sst_data():
@@ -48,63 +54,48 @@ def test_roundtrip_own_writer_reader():
         sst.write_sst([(b"b", b"1"), (b"a", b"2")])  # "Keys must be added in order"
 
 
-def _ref_extras(ref_lib):
-    ref_lib.okv_write_sst.restype = C.c_int
-    ref_lib.okv_write_sst.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_void_p, C.c_char_p, C.c_void_p, C.c_char_p, C.c_size_t]
-    ref_lib.okv_ingest_sst.restype = C.c_int
-    ref_lib.okv_ingest_sst.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_char_p, C.c_size_t]
-    return ref_lib
-
-
-def test_reads_files_written_by_the_reference(ref_lib):
-    import numpy as np
-    lib = _ref_extras(ref_lib)
-    tmp = tempfile.mkdtemp(dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
-    for n, seed in ((1, 11), (50, 12), (4000, 13)):
-        kv = _kv(n, seed, max_v=2000)
-        koff = np.zeros(len(kv) + 1, dtype=np.uint64)
-        voff = np.zeros(len(kv) + 1, dtype=np.uint64)
-        np.cumsum([len(k) for k, _ in kv], out=koff[1:])
-        np.cumsum([len(v) for _, v in kv], out=voff[1:])
-        path = os.path.join(tmp, "ref%d.sst" % n)
-        err = C.create_string_buffer(256)
-        rc = lib.okv_write_sst(path.encode(), len(kv), b"".join(k for k, _ in kv) + b"\0", koff.ctypes.data,
-                               b"".join(v for _, v in kv) + b"\0", voff.ctypes.data, err, 256)
-        assert rc == 0, err.value
-        entries, props = sst.read_sst(open(path, "rb").read())
+def test_reads_files_written_by_the_reference():
+    """tests/golden/ref_written_<n>.sst: what the reference's SstFileWriter wrote for _kv(n, seed, max_v)
+    (oracle/gen_golden.py)"""
+    for n, seed, max_v in REF_WRITTEN:
+        kv = _kv(n, seed, max_v=max_v)
+        entries, props = sst.read_sst(open(os.path.join(GOLDEN_DIR, "ref_written_%d.sst" % n), "rb").read())
         assert [(k, t, v) for k, _, t, v in entries] == [(k, 1, v) for k, v in kv]
         assert props["external_version"] == 2 and props["global_seqno"] == 0 and props["num_entries"] == len(kv)
 
 
-def test_reference_ingests_files_written_here(ref_lib):
-    from oracle import okv
-    lib = _ref_extras(ref_lib)
-    tmp = tempfile.mkdtemp(dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
-    for n, seed in ((1, 21), (200, 22), (5000, 23)):
-        kv = _kv(n, seed, max_v=1500)
-        path = os.path.join(tmp, "ours%d.sst" % n)
-        open(path, "wb").write(sst.write_sst(kv))
-        db = okv.Okv(lib)
-        err = C.create_string_buffer(256)
-        rc = lib.okv_ingest_sst(db.h, path.encode(), 1, err, 256)
-        assert rc == 0, err.value
-        assert db.latest_seq() == 0  # ingest into an empty DB does not consume sequence numbers
-        assert db.scan() == kv
-        for k, v in kv[:: max(1, len(kv) // 50)]:
-            assert db.get(k) == (0, v)
+def ingest_inputs(n, seed):
+    """test_reference_ingests_files_written_here's two files: kv, then an overlapping update of every third key"""
+    kv = _kv(n, seed, max_v=1500)
+    return kv, [(k, b"second:" + v[:5]) for k, v in kv[::3]]
+
+
+INGESTED = ((1, 21), (200, 22), (5000, 23))
+
+
+def test_reference_ingests_files_written_here():
+    """What the reference's DB::IngestExternalFile made of files written here, recorded by oracle/gen_golden.py in
+    tests/golden/differential.json for these exact bytes (a writer that changes them has to be checked again)."""
+    rec = G.load("differential.json")["sst_ingest"]
+    for n, seed in INGESTED:
+        kv, kv2 = ingest_inputs(n, seed)
+        f1, f2 = sst.write_sst(kv), sst.write_sst(kv2)
+        r = rec[str(n)]
+        assert [r["file"], r["file2"]] == [G.sha256(f1), G.sha256(f2)], n
+        assert r["rc"] == 0, r["error"]
+        assert r["seq"] == 0  # ingest into an empty DB does not consume sequence numbers
+        assert r["scan"] == G.digest(kv)
+        assert r["get"] == G.digest([(0, v) for k, v in kv[:: max(1, len(kv) // 50)]])
         # an overlapping second ingest is given global sequence number last+1 (rocksdb_assumption_test.cpp:272-283)
-        kv2 = [(k, b"second:" + v[:5]) for k, v in kv[::3]]
-        path2 = os.path.join(tmp, "ours%d_b.sst" % n)
-        open(path2, "wb").write(sst.write_sst(kv2))
-        assert lib.okv_ingest_sst(db.h, path2.encode(), 1, err, 256) == 0, err.value
-        assert db.latest_seq() == 1
+        assert r["rc2"] == 0, r["error2"]
+        assert r["seq2"] == 1
         want = dict(kv)
         want.update(kv2)
-        assert db.scan() == sorted(want.items())
+        assert r["scan2"] == G.digest(sorted(want.items()))
         # (move_files = false: RocksDB stamps the sequence number into ITS copy; the file written here is untouched)
-        entries, props = sst.read_sst(open(path2, "rb").read())
+        assert r["file2_after"] == G.sha256(f2)
+        entries, props = sst.read_sst(f2)
         assert props["global_seqno"] == 0 and [(k, v) for k, _, _, v in entries] == kv2
-        db.close()
 
 
 def test_shard_file_helpers_host_half():

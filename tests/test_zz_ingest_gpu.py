@@ -1,15 +1,14 @@
 """GPU parity of rsp_ingest_sorted (DB::IngestExternalFile for a sorted set of Puts) against the reference's own RocksDB
-ingesting the SAME file (written by rocksplicator_b200/sst.py): contents, reads and the sequence-number rules of
-rocksdb_replicator/tests/rocksdb_assumption_test.cpp:248-283.  Runs last (file name) — it is the newest entry point.
+ingesting the SAME file (written by rocksplicator_b200/sst.py; its answers recorded by oracle/gen_golden.py): contents,
+reads and the sequence-number rules of rocksdb_replicator/tests/rocksdb_assumption_test.cpp:248-283.  Runs last (file
+name) — it is the newest entry point.
 """
-import ctypes as C
 import os
 import random
-import tempfile
 
 import pytest
 
-from oracle import okv
+import golden_util as G
 from rocksplicator_b200 import sst
 from rocksplicator_b200.write_batch import WriteBatch
 
@@ -30,24 +29,38 @@ def _kv(n, seed, lo=0, hi=1 << 30, max_v=300):
     return [(k, rnd.randbytes(rnd.randrange(0, max_v))) for k in keys]
 
 
-class RefDb:
-    """the reference's RocksDB ingesting the files our writer produces (None when oracle/_ref was not built)"""
+def ingest_inputs():
+    """the files and WriteBatches of test_ingest_sequence_rules_and_contents, in the order they are applied"""
+    f1 = _kv(3000, 1, lo=0, hi=1 << 20)
+    wb1 = WriteBatch().put(f1[10][0], b"overwritten").delete(f1[11][0]).put(b"k-new", b"v").data()
+    f2 = _kv(500, 2, lo=1 << 28, hi=1 << 29)
+    f3 = sorted(dict([(k, b"third:" + v[:4]) for k, v in f1[::7]] + [(f1[11][0], b"back")]).items())
+    f4 = [(f1[5][0], b"refused")]
+    wb2 = WriteBatch().put(f3[0][0], b"after").delete(f2[0][0]).data()
+    return f1, wb1, f2, f3, f4, wb2
+
+
+class RecordedRef:
+    """The reference's RocksDB given the same files (the bytes our writer produces) and WriteBatches: its answers, in
+    call order, as oracle/gen_golden.py recorded them in tests/golden/differential.json"""
 
     def __init__(self):
-        self.lib = okv.load_ref()
-        self.lib.okv_ingest_sst.restype = C.c_int
-        self.lib.okv_ingest_sst.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_char_p, C.c_size_t]
-        self.db = okv.Okv(self.lib)
-        self.tmp = tempfile.mkdtemp(dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
-        self.n = 0
+        self.rec = iter(G.load("differential.json")["ingest_gpu"])
+
+    def _next(self, kind, *inputs):
+        r = next(self.rec)
+        assert r[:len(inputs) + 1] == [kind, *inputs], (r, kind, inputs)
+        return r[len(inputs) + 1:]
 
     def ingest(self, kv, allow=True):
-        self.n += 1
-        path = os.path.join(self.tmp, "f%d.sst" % self.n)
-        with open(path, "wb") as f:
-            f.write(sst.write_sst(kv))
-        err = C.create_string_buffer(256)
-        return self.lib.okv_ingest_sst(self.db.h, path.encode(), 1 if allow else 0, err, 256)
+        return self._next("ingest", G.sha256(sst.write_sst(kv)), int(allow))[0]
+
+    def apply(self, batch, ts):
+        return self._next("apply", G.sha256(batch), ts)[0]
+
+    def check(self):
+        """-> [latest_seq, digest of the full scan]"""
+        return self._next("check")
 
 
 def _check(s, want, seq, ref):
@@ -56,55 +69,42 @@ def _check(s, want, seq, ref):
     keys = list(want)[:: max(1, len(want) // 64)] + [b"k-absent", b"zzz"]
     got = s.multi_get(keys)
     assert got == [(0, want[k]) if k in want else (1, None) for k in keys]
-    if ref is not None:
-        assert ref.db.latest_seq() == seq
-        assert ref.db.scan() == sorted(want.items())
+    assert ref.check() == [seq, G.digest(sorted(want.items()))]
 
 
 def test_ingest_sequence_rules_and_contents(eng):
-    ref = RefDb() if okv.ref_available() else None
+    ref = RecordedRef()
     s = eng.open_shard("ingest-a")
     want = {}
+    f1, wb1, f2, f3, f4, wb2 = ingest_inputs()
     # 1. into an empty shard: no sequence number is consumed
-    f1 = _kv(3000, 1, lo=0, hi=1 << 20)
     assert s.ingest(f1) == 0
-    if ref: assert ref.ingest(f1) == 0
+    assert ref.ingest(f1) == 0
     want.update(f1)
     _check(s, want, 0, ref)
     # 2. writes on top, then a file whose range lies beyond everything: still no bump
-    wb = WriteBatch()
-    wb.put(f1[10][0], b"overwritten")
-    wb.delete(f1[11][0])
-    wb.put(b"k-new", b"v")
-    assert s.apply(wb.data(), 1234) == 0
-    if ref: assert ref.db.apply(wb.data(), 1234) == 0
+    assert s.apply(wb1, 1234) == 0
+    assert ref.apply(wb1, 1234) == 0
     want[f1[10][0]] = b"overwritten"
     del want[f1[11][0]]
     want[b"k-new"] = b"v"
     _check(s, want, 3, ref)
-    f2 = _kv(500, 2, lo=1 << 28, hi=1 << 29)
     assert s.ingest(f2) == 0
-    if ref: assert ref.ingest(f2) == 0
+    assert ref.ingest(f2) == 0
     want.update(f2)
     _check(s, want, 3, ref)
     # 3. an overlapping file is newer than everything and takes sequence number last+1
-    f3 = [(k, b"third:" + v[:4]) for k, v in f1[::7]] + [(f1[11][0], b"back")]
-    f3 = sorted(dict(f3).items())
     assert s.ingest(f3) == 0
-    if ref: assert ref.ingest(f3) == 0
+    assert ref.ingest(f3) == 0
     want.update(f3)
     _check(s, want, 4, ref)
     # 4. ... and is refused when global sequence numbers are not allowed; nothing changes
-    f4 = [(f1[5][0], b"refused")]
     assert s.ingest(f4, allow_global_seqno=False) == 4
-    if ref: assert ref.ingest(f4, allow=False) != 0
+    assert ref.ingest(f4, allow=False) != 0
     _check(s, want, 4, ref)
     # 5. later writes and a full compaction see the ingested data like any other
-    wb = WriteBatch()
-    wb.put(f3[0][0], b"after")
-    wb.delete(f2[0][0])
-    assert s.apply(wb.data(), 1234) == 0
-    if ref: assert ref.db.apply(wb.data(), 1234) == 0
+    assert s.apply(wb2, 1234) == 0
+    assert ref.apply(wb2, 1234) == 0
     want[f3[0][0]] = b"after"
     del want[f2[0][0]]
     _check(s, want, 6, ref)
@@ -115,7 +115,7 @@ def test_ingest_sequence_rules_and_contents(eng):
     assert s.ingest([(b"a", b"1"), (b"a", b"2")]) == 4
     _check(s, want, 6, ref)
     s.close()
-    if ref: ref.db.close()
+    assert next(ref.rec, None) is None
 
 
 def test_ingest_fixed_shape_serves_the_fast_path(eng):

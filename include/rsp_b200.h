@@ -237,6 +237,9 @@ int rsp_ingest_sorted(rsp_shard* s, size_t n, const uint8_t* keys, const uint64_
 int rsp_multi_get_device(rsp_engine* e, size_t n, const uint32_t* d_shard_ix, const uint8_t* d_keys,
                          uint32_t klen, uint8_t* d_vals, uint32_t val_stride, uint32_t* d_vlen,
                          int32_t* d_st, void* stream);
+/* The raw form of rsp_multi_scan: d_st / the vlen markers as described there, untranslated.  A scan whose shard id is
+ * >= max_shards or names a shard that is not open answers d_st = RSP_INVALID_ARGUMENT, d_n_out = 0 and writes no output
+ * bytes (as rsp_multi_get_device answers such lookups); the other scans of the launch are unaffected. */
 int rsp_multi_scan_device(rsp_engine* e, size_t n, const uint32_t* d_shard_ix, const uint8_t* d_keys,
                           uint32_t klen, uint32_t max_entries, uint8_t* d_out, uint64_t out_stride,
                           uint32_t* d_n_out, int32_t* d_st, void* stream);

@@ -7,6 +7,8 @@ The .so is git-ignored but travels to the GPU box with the gpurun snapshot.
 import os
 import subprocess
 import sys
+import tempfile
+import zlib
 from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -84,10 +86,18 @@ def build_host(force=False, verbose=False):
             print(" ".join(cmd))
         subprocess.check_call(cmd)
 
+    deps.append(os.path.join(os.path.dirname(HERE), "include", "rsp_b200.h"))  # (gpu_db.h includes the C ABI)
     if force or _stale(HOST_SO, deps + [OUT]):
         run([cxx] + flags + ["-shared", "-o", HOST_SO] + srcs + ["-L", HERE, "-lrsp_b200", "-Wl,-rpath,$ORIGIN"])
     tsrc = os.path.join(os.path.dirname(HERE), "tests", "cpp", "host_tests.cpp")
-    if force or _stale(HOST_TESTS, [tsrc, HOST_SO] + deps):
-        run([cxx] + flags + ["-o", HOST_TESTS, tsrc, "-L", HERE, "-lrsp_host", "-lrsp_b200",
-                             "-Wl,-rpath," + HERE])
-    return HOST_SO, HOST_TESTS
+    tdeps = [tsrc, HOST_SO] + deps
+    exe = HOST_TESTS
+    if (force or _stale(exe, tdeps)) and not os.access(os.path.dirname(exe), os.W_OK):
+        # the suite runs from a checkout whose tests/ is read-only: a test binary that has to be (re)linked goes to a
+        # per-user directory outside the tree
+        exe = os.path.join(tempfile.gettempdir(), "rsp_host_tests_%d_%08x" % (os.getuid(), zlib.crc32(HERE.encode())),
+                           "host_tests")
+        os.makedirs(os.path.dirname(exe), exist_ok=True)
+    if force or _stale(exe, tdeps):
+        run([cxx] + flags + ["-o", exe, tsrc, "-L", HERE, "-lrsp_host", "-lrsp_b200", "-Wl,-rpath," + HERE])
+    return HOST_SO, exe

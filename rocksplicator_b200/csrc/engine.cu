@@ -1550,7 +1550,7 @@ static void iter_fetch(rsp_iter* it, const std::string* key, bool exclusive, boo
     ScanArgs a;
     a.shards = nullptr; a.views = it->d_view; a.shard_ix = nullptr; a.keys = d + o_key; a.koff = (const u64*)d;
     a.klen_fixed = 0; a.flags = d + 16; a.max_entries = (u32)it->want; a.out = d + o_out; a.out_stride = it->stride;
-    a.n_out = (u32*)(d + 32); a.st = (i32*)(d + 36); a.n = 1;
+    a.n_out = (u32*)(d + 32); a.st = (i32*)(d + 36); a.n = 1; a.max_shards = 0;
     launch_multi_scan(a, e->st);
     e->launches++;
     u32 res[2];
@@ -2833,6 +2833,7 @@ int rsp_multi_scan(rsp_engine* e, size_t n, const uint32_t* shard_ix, const uint
   a.shards = e->d_shards; a.views = nullptr; a.shard_ix = (const u32*)d; a.keys = d + o_keys;
   a.koff = (const u64*)(d + o_koff); a.klen_fixed = 0; a.flags = nullptr; a.max_entries = max_entries;
   a.out = d + o_out; a.out_stride = out_stride; a.n_out = (u32*)(d + o_nout); a.st = (i32*)(d + o_st); a.n = (u32)n;
+  a.max_shards = e->cfg.max_shards;
   CUDA_OK(cudaEventRecord(e->ev0, e->st));
   launch_multi_scan(a, e->st);
   e->launches++;
@@ -2896,7 +2897,7 @@ int rsp_multi_scan_device(rsp_engine* e, size_t n, const uint32_t* d_shard_ix, c
   ScanArgs a;
   a.shards = e->d_shards; a.views = nullptr; a.shard_ix = d_shard_ix; a.keys = d_keys; a.koff = nullptr;
   a.klen_fixed = klen; a.flags = nullptr; a.max_entries = max_entries; a.out = d_out; a.out_stride = out_stride;
-  a.n_out = d_n_out; a.st = d_st; a.n = (u32)n;
+  a.n_out = d_n_out; a.st = d_st; a.n = (u32)n; a.max_shards = e->cfg.max_shards;
   {
     std::lock_guard<std::mutex> g(e->mu);
     cudaStream_t rs = stream ? (cudaStream_t)stream : e->st;

@@ -952,8 +952,20 @@ __device__ __forceinline__ void multi_scan_body(const ScanArgs& a) {
   if (a.views) {
     runs = a.views[q].runs; n_runs = a.views[q].n_runs; merge_op = a.views[q].merge_op;
   } else {
-    const ShardDev* sd = a.shards + a.shard_ix[q];
+    // unknown / closed shard: InvalidArgument, no output bytes.  An unknown id reads slot 0 (never past the table), so
+    // that `live` is loaded together with the fields below rather than ahead of them: an extra dependent load at the
+    // head of every scan costs the short-lived scan warps a third of their rate
+    const u32 six = a.shard_ix[q];
+    const bool known = six < a.max_shards;
+    const ShardDev* sd = a.shards + (known ? six : 0u);
     runs = sd->runs; n_runs = sd->n_runs; merge_op = sd->merge_op;
+    if (!known || !sd->live) {
+      if (lane == 0) {
+        a.n_out[q] = 0;
+        a.st[q] = 4;
+      }
+      return;
+    }
   }
   const u8* kp;
   u32 klen;

@@ -187,6 +187,7 @@ struct ScanArgs {
   u32* n_out;
   i32* st;
   u32 n;
+  u32 max_shards;           // with `shards`: ids >= this (and closed shards) answer InvalidArgument
 };
 void launch_multi_scan(const ScanArgs& a, cudaStream_t s);
 

@@ -45,6 +45,13 @@ def test_parity_suite_under_emulation(emul):
     assert " passed" in out and "failed" not in out
 
 
+def test_device_forms_under_emulation(emul):
+    """tests/test_device_forms_gpu.py (the device-pointer entry points at every buffer shape, raw scan statuses, staged
+    ticks) against the emulation"""
+    out = _pytest_under_emulation(emul[0], {}, ["tests/test_device_forms_gpu.py"], timeout=900)
+    assert " passed" in out and "failed" not in out
+
+
 def test_router_over_two_emulated_devices(emul):
     """tests/test_router_gpu.py (two engines behind one router, maintenance on both) against the emulation"""
     out = _pytest_under_emulation(emul[0], {"RSP_EMUL_DEVICES": "2"}, ["tests/test_router_gpu.py"])

@@ -275,6 +275,33 @@ void rsp_debug_combiner_stats(rsp_engine* e, int which, uint64_t out[9]);
  * bytes free inside the slabs} */
 void rsp_debug_arena(rsp_engine* e, uint64_t out[4]);
 
+/* diagnostics, not part of the product path: read back run r of a shard (0 = newest) as flush and compaction built it,
+ * for tests that check a run's structure entry by entry.  Synchronises the engine stream; changes no state.
+ * info gets the engine's descriptor of the run (host), the descriptor the readers use (ShardDev.runs[r] and
+ * ShardDev.n_runs, copied back from the device), the run's row of the per-run fast descriptors and, for r == 0, the
+ * shard's fast descriptor (zero otherwise).  A run is identified by host.heap, its heap's device address.  With all of
+ * heap, ent_off, blk_pfx and hslots NULL only info is filled (the sizes).  Otherwise *info must hold what an earlier
+ * call returned for this run, and the non-NULL buffers receive a copy of heap (host.heap_units x 16 bytes), ent_off
+ * (host.n_ent x 4), blk_pfx (host.n_blocks x 8) and hslots (host.n_buckets x 32); RSP_BUSY and nothing copied when run
+ * r has been replaced since (a background merge).  RSP_NOT_FOUND when the shard has no run r. */
+typedef struct rsp_debug_run_desc { /* RunDev (format.cuh) */
+  uint64_t heap, ent_off, hslots, blk_pfx; /* device addresses */
+  uint32_t n_ent, n_buckets, ord_bits, uniform_units, n_blocks, heap_units, flags, kv_len;
+} rsp_debug_run_desc;
+typedef struct rsp_debug_fast_desc { /* ShardFast (format.cuh) */
+  uint64_t run0_heap, run0_hslots;
+  uint32_t n_buckets, meta, mt_count, merge_op;
+} rsp_debug_fast_desc;
+typedef struct rsp_debug_run_info {
+  uint32_t n_runs;     /* runs of the shard (host) */
+  uint32_t dev_n_runs; /* ShardDev.n_runs on the device */
+  rsp_debug_run_desc host, dev;
+  rsp_debug_fast_desc fast_run; /* the per-run fast descriptor of run r on the device */
+  rsp_debug_fast_desc fast;     /* r == 0: the shard's ShardFast on the device */
+} rsp_debug_run_info;
+int rsp_debug_run(rsp_shard* s, uint32_t r, rsp_debug_run_info* info, uint8_t* heap, uint32_t* ent_off,
+                  uint64_t* blk_pfx, uint32_t* hslots);
+
 const char* rsp_version(void);
 
 #ifdef __cplusplus

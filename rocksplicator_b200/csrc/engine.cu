@@ -2253,8 +2253,10 @@ int rsp_ingest_sorted(rsp_shard* s, size_t n, const uint8_t* keys, const uint64_
   if (rc == RSP_OK) {
     compact_shards(e, {tmp}, false);
     if (tmp->runs.size() > 1) compact_shards(e, {tmp}, true);
+    std::shared_ptr<Run> in;
     if (!tmp->runs.empty()) {
-      s->runs.insert(s->runs.begin(), tmp->runs[0]);
+      in = tmp->runs[0];
+      s->runs.insert(s->runs.begin(), in);
       tmp->runs.clear();
     }
     if (overlap) {
@@ -2262,6 +2264,11 @@ int rsp_ingest_sorted(rsp_shard* s, size_t n, const uint8_t* keys, const uint64_
       s->h.last_seq = seq;
       s->h.pub_seq = seq;
       s->last_seq.store(seq, std::memory_order_release);
+    }
+    if (in) {  // (before the descriptor upload below: no reader sees the run yet)
+      launch_set_run_seq(in->heap, in->ent_off, in->n_ent, s->last_seq.load(), e->st);
+      CUDA_OK(cudaGetLastError());
+      e->launches += 1;
     }
     upload_shard(e, s);
     note_mutation(e);
@@ -2985,6 +2992,38 @@ void rsp_debug_arena(rsp_engine* e, uint64_t out[4]) {
   out[1] = e->arena.reserved;     // bytes reserved from the device (slabs)
   out[2] = e->arena.blocks.size();  // blocks, free and used
   out[3] = e->arena.free_bytes;   // free inside the slabs
+}
+
+int rsp_debug_run(rsp_shard* s, uint32_t r, rsp_debug_run_info* info, uint8_t* heap, uint32_t* ent_off,
+                  uint64_t* blk_pfx, uint32_t* hslots) {
+  try {
+  if (!s || !info) return RSP_INVALID_ARGUMENT;
+  rsp_engine* e = s->eng;
+  std::lock_guard<std::mutex> g(e->mu);
+  if (r >= s->runs.size()) return RSP_NOT_FOUND;
+  CUDA_OK(cudaSetDevice(e->device));
+  static_assert(sizeof(rsp_debug_run_desc) == sizeof(RunDev) && sizeof(rsp_debug_fast_desc) == sizeof(ShardFast), "layout");
+  const Run& run = *s->runs[r];
+  // the buffers were sized from an earlier call: copy only into buffers sized for THIS run
+  if ((heap || ent_off || blk_pfx || hslots) && info->host.heap != (uint64_t)run.heap) return RSP_BUSY;
+  memset(info, 0, sizeof(*info));
+  const RunDev hd = run.dev();
+  memcpy(&info->host, &hd, sizeof(RunDev));
+  info->n_runs = (u32)s->runs.size();
+  const ShardDev* d = e->d_shards + s->index;
+  CUDA_OK(cudaMemcpyAsync(&info->dev_n_runs, &d->n_runs, 4, cudaMemcpyDeviceToHost, e->st));
+  CUDA_OK(cudaMemcpyAsync(&info->dev, &d->runs[r], sizeof(RunDev), cudaMemcpyDeviceToHost, e->st));
+  CUDA_OK(cudaMemcpyAsync(&info->fast_run, e->d_fast_runs + (size_t)s->index * RSP_MAX_RUNS + r, sizeof(ShardFast),
+                          cudaMemcpyDeviceToHost, e->st));
+  if (r == 0) CUDA_OK(cudaMemcpyAsync(&info->fast, e->d_fast + s->index, sizeof(ShardFast), cudaMemcpyDeviceToHost, e->st));
+  if (heap && run.heap_units) CUDA_OK(cudaMemcpyAsync(heap, run.heap, (size_t)run.heap_units * 16, cudaMemcpyDeviceToHost, e->st));
+  if (ent_off && run.n_ent) CUDA_OK(cudaMemcpyAsync(ent_off, run.ent_off, (size_t)run.n_ent * 4, cudaMemcpyDeviceToHost, e->st));
+  if (blk_pfx && run.n_blocks) CUDA_OK(cudaMemcpyAsync(blk_pfx, run.blk_pfx, (size_t)run.n_blocks * 8, cudaMemcpyDeviceToHost, e->st));
+  if (hslots && run.n_buckets)
+    CUDA_OK(cudaMemcpyAsync(hslots, run.hslots, (size_t)run.n_buckets * RUN_BUCKET_SLOTS * 4, cudaMemcpyDeviceToHost, e->st));
+  CUDA_OK(cudaStreamSynchronize(e->st));
+  return RSP_OK;
+  } catch (...) { return abi_caught(); }
 }
 
 void rsp_debug_combiner_stats(rsp_engine* e, int which, uint64_t out[9]) {

@@ -618,6 +618,19 @@ void launch_upload_shards(const ShardUpload* d_up, u32 n, ShardDev* shards, Shar
   k_upload_shards<<<n, 128, 0, s>>>(d_up, shards, fast, fast_runs, mt_filter);
 }
 
+// An ingested run takes the sequence number of the ingest, all its entries alike: the scratch shard it was built on
+// numbered them 1..n, which may be below the versions of the same keys in older runs.
+__global__ void __launch_bounds__(256) k_set_run_seq(u8* heap, const u32* ent_off, u32 n, u64 seq) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  u64* st = reinterpret_cast<u64*>(heap + (u64)ent_off[i] * 16u);
+  *st = (seq << 8) | (*st & 0xffull);
+}
+void launch_set_run_seq(u8* heap, const u32* ent_off, u32 n, u64 seq, cudaStream_t s) {
+  if (!n) return;
+  k_set_run_seq<<<(n + 255) / 256, 256, 0, s>>>(heap, ent_off, n, seq);
+}
+
 void launch_compact_sort(const CompactJob* d_jobs, const CompactJob* h_jobs, u32 n_jobs, cudaStream_t s) {
   if (!n_jobs) return;
   u32 max_len = 0, max_sort = 0, max_tiles = 0;

@@ -237,6 +237,7 @@ void launch_compact_sort(const CompactJob* d_jobs, const CompactJob* h_jobs, u32
 void launch_compact_size(const CompactJob* d_jobs, u32 n_jobs, cudaStream_t s);
 void launch_compact_write(const CompactJob* d_jobs, u32 n_jobs, u32 max_items, cudaStream_t s);
 // zero the hash index of every job's output run (out_hslots, out_n_buckets buckets): one launch for the whole batch
+void launch_set_run_seq(u8* heap, const u32* ent_off, u32 n, u64 seq, cudaStream_t s);
 void launch_zero_out_hslots(const CompactJob* d_jobs, u32 n_jobs, u32 max_buckets, cudaStream_t s);
 
 // ---- batched descriptor upload ------------------------------------------------------------------------

@@ -107,6 +107,7 @@ EXPORTS = {
     "rsp_debug_last_pending": (C.c_uint32, [C.c_void_p, C.c_void_p, C.c_uint32]),
     "rsp_debug_combiner_stats": (None, [C.c_void_p, C.c_int, C.c_void_p]),
     "rsp_debug_arena": (None, [C.c_void_p, C.c_void_p]),
+    "rsp_debug_run": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE — differential fuzzer: the engine (compiled against the CPU emulation, tests/emul) against the
 oracle port on random streams: every merge operator, variable and fixed key shapes, tiny and default write buffers
 (forced flushes), flush / compaction at random points, single applies and multi-shard ticks (rsp_apply_many),
-Get / MultiGet / full scans / iterator walks compared after every few batches.  GPU time is too scarce for hundreds of
+Get / MultiGet / full scans / iterator walks compared after every few batches, every run of a shard checked by
+tests/test_compaction_gpu.py's validate_shard after each explicit flush and compaction.  GPU time is too scarce for hundreds of
 seeds; the emulation runs them for free.  `python tests/emul/fuzz_engine_vs_port.py FIRST LAST [env VAR=1 ...]`.
 A short range runs in tests/test_emul_cpu.py.
 """
@@ -17,6 +18,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 from oracle import okv  # noqa: E402
 from rocksplicator_b200 import engine  # noqa: E402
 from streams import random_stream  # noqa: E402
+from test_compaction_gpu import validate_shard  # noqa: E402
 
 
 def iter_walk(db, keys, seed):
@@ -214,8 +216,10 @@ def one_seed(eng, port, seed):
             if not bad:
                 if r < (0.10 if heavy else 0.05):
                     shards[x].flush()
+                    validate_shard(shards[x], merge_op=mop)
                 elif r < (0.13 if heavy else 0.08):
                     shards[x].compact()
+                    validate_shard(shards[x], merge_op=mop)
             if rng.random() < 0.08:
                 compare(shards[x], oracles[x], keys, (seed, i, x))
             if rng.random() < 0.06 and len(live) < 6:
@@ -242,8 +246,10 @@ def one_seed(eng, port, seed):
             assert got == [oracles[x].get(k) for x, k in pick], (seed, "cross-shard multi_get")
         for x in range(n_shards):
             compare(shards[x], oracles[x], keys, (seed, "end", x))
+            validate_shard(shards[x], merge_op=mop)
             if not bad:
                 shards[x].compact()
+                validate_shard(shards[x], merge_op=mop)
                 compare(shards[x], oracles[x], keys, (seed, "compacted", x))
     finally:
         for ia, ib in live:

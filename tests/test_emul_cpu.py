@@ -52,6 +52,13 @@ def test_device_forms_under_emulation(emul):
     assert " passed" in out and "failed" not in out
 
 
+def test_compaction_runs_under_emulation(emul):
+    """tests/test_compaction_gpu.py (every flushed and compacted run validated and compared with the host model of the
+    merge rules) against the emulation"""
+    out = _pytest_under_emulation(emul[0], {}, ["tests/test_compaction_gpu.py"], timeout=1500)
+    assert " passed" in out and "failed" not in out
+
+
 def test_router_over_two_emulated_devices(emul):
     """tests/test_router_gpu.py (two engines behind one router, maintenance on both) against the emulation"""
     out = _pytest_under_emulation(emul[0], {"RSP_EMUL_DEVICES": "2"}, ["tests/test_router_gpu.py"])
